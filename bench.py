@@ -30,6 +30,8 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark runs from the tree build() left, which may be read-only: no bytecode caches in it
+sys.dont_write_bytecode = True
 
 N_MEMBERS = 1_000_000
 TICKS_PER_STEP = 2048
@@ -145,7 +147,8 @@ def _oracle():
     """oracle_binding without building or loading anything of the product."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import __graft_entry__ as ge
-    ge.build_oracle()
+    if not os.path.exists(ge.LIBORACLE):     # build() made it; the tree is not written otherwise
+        ge.build_oracle()
     import oracle_binding
     return oracle_binding
 
@@ -230,6 +233,40 @@ def workload_shape(args, world: int) -> tuple:
     return args.members, args.members + 2 * total_steps + 8, False
 
 
+DUMP_BYTES = 64 << 20       # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir: str, pool, with_members: bool) -> None:
+    """What the last timed step leaves a caller with, as float64 .npy files (every value is an
+    integer below 2**53, so float64 holds it exactly):
+      stats.npy       Stats() in the order of consul_b200.pool.Pool.stats(), without active_rows
+                      (how many rows left the kernels' idle fast path: a scheduling count, not a result)
+      state_hash.npy  the 256-bit state digest as eight 32-bit words, high word of each 64-bit lane first
+      members.npy     Members() as member 0 reports it, one row (id, status, incarnation, rank) per
+                      member; beyond the byte budget, a fixed seeded sample of rows in id order
+    Members() of a sharded pool would pull every row through rank 0, so it is left out there.  Every
+    rank of a sharded pool must issue the same reads; the ranks other than 0 pass out_dir=None.
+    (The reference arm's state is that of the ticks it executed: reproducible when its line's
+    cpu_baseline.sample says every tick was.)"""
+    import numpy as np
+    st = pool.stats()
+    st.pop("active_rows")
+    stats = [float(x) for v in st.values() for x in (v if isinstance(v, list) else [v])]
+    digest = [float(w) for h in pool.state_hash() for w in (h >> 32, h & 0xFFFFFFFF)]
+    members = np.array(pool.members(0), dtype=np.float64) if with_members else None
+    if out_dir is None:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "stats.npy"), np.array(stats, dtype=np.float64))
+    np.save(os.path.join(out_dir, "state_hash.npy"), np.array(digest, dtype=np.float64))
+    if members is not None:
+        max_rows = (DUMP_BYTES - (1 << 20)) // members.itemsize // 4
+        if len(members) > max_rows:
+            rows = np.sort(np.random.default_rng(SEED).choice(len(members), max_rows, replace=False))
+            members = members[rows]
+        np.save(os.path.join(out_dir, "members.npy"), members)
+
+
 def mapped_native_libs() -> list:
     out = set()
     try:
@@ -276,6 +313,8 @@ def run_reference(args, rank: int, world: int):
         s_, d_ = one_step()
         secs += s_
         executed += d_
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o, with_members=True)
     n_now = o.stats()["n_members"]
     val = float(n_now) * ticks * args.steps / secs / 1e6
     exact = executed == ticks * args.steps
@@ -369,6 +408,8 @@ def main():
     ap.add_argument("--skip-hbm-point", action="store_true")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -465,6 +506,8 @@ def main():
     c1 = pool.sched_counts()
     d = stat_delta(s0, s1)
     sc = {k: c1[k] - c0[k] for k in c1}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if rank == 0 else None, pool, with_members=not sharded)
 
     # ticks-to-full-convergence of one cascade (untimed, exact tick recorded on the device)
     x = pool.member_add()

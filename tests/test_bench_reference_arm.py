@@ -23,17 +23,25 @@ def test_oracle_presets_equal_libgsim_presets(hostemu_lib):
             assert getattr(a, name) == getattr(b, name), (preset, name)
 
 
-def test_reference_arm_runs_without_the_product_library():
+def test_reference_arm_runs_without_the_product_library(tmp_path):
     env = dict(os.environ, OMP_NUM_THREADS="1", GSIM_REF_BUDGET_S="20")     # as under torchrun
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
-                        "--warmup", "1", "--members", "30000", "--ticks", "160"], capture_output=True, text=True,
-                       timeout=300, env=env, cwd=ROOT)
+                        "--warmup", "1", "--members", "30000", "--ticks", "160", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=300, env=env, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
     assert line["impl"] == "reference" and line["native_so_loaded"] == ["oracle/liboracle.so"]
     assert line["config"]["ticks_per_step"] == 160 and line["config"]["members"] == 30000
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["value"] == line["value"] > 0
+    # --dump-outputs: the state the last timed step left, the one the line's digest was taken from
+    import numpy as np
+    words = np.load(tmp_path / "state_hash.npy")
+    assert words.dtype == np.float64 and words.shape == (8,)
+    assert "%016x" % (int(words[0]) << 32 | int(words[1])) == line["digest"]
+    members = np.load(tmp_path / "members.npy")
+    assert members.shape == (30000 + 1 + 2, 4) and (members[:, 0] == np.arange(len(members))).all()
+    assert np.load(tmp_path / "stats.npy").dtype == np.float64
     # the config object is produced by the one function the repo arm uses
     sys.path.insert(0, ROOT)
     import bench
