@@ -783,6 +783,7 @@ extern "C" int gsim_pool_create(const gsim_config* cfg, gsim_pool** out) {
   g.seed_lo = (uint32_t)cfg->seed;
   g.seed_hi = (uint32_t)(cfg->seed >> 32);
   g.flags = cfg->flags;
+  if (getenv("GSIM_NO_FAST_GOSSIP") != nullptr) g.flags |= GSIM_FLAG_NO_FAST_GOSSIP;  // measurement knob
   g.evlog_cap = evcap;
   g.world = cfg->world_size;
   g.rank = cfg->rank;

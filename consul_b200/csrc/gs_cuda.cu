@@ -171,6 +171,17 @@ __device__ __noinline__ void gs_row_step_call(const GsDev* dp, const GsGlobals* 
   gs_row_step(*dp, *gp, i, t, t % gp->GI, inb, sink);
 }
 
+// The fast gossip tier (gs_fast_gossip), out of line for the same reason: its own register budget, and a
+// few hundred instructions that stay resident in the instruction cache while a cascade tick drains its
+// queue.  Returns false, having written nothing, for a member that needs the generic step.
+template <bool COORDS>
+__device__ __noinline__ bool gs_fast_gossip_call(const GsDev* dp, const GsGlobals* gp, uint32_t i, uint32_t t,
+                                                 uint32_t gslot, uint32_t inb, bool due_now, uint32_t* s_stat,
+                                                 uint32_t* s_heard, uint32_t* s_q) {
+  DevSinkT<COORDS> sink{s_stat, s_heard, s_q};
+  return gs_fast_gossip(*dp, *gp, sink, i, t, gslot, inb, due_now);
+}
+
 // Persistent, warp-centric tick.  Every warp owns a CONTIGUOUS chunk of tiles (128 members
 // each); because ticker phases are dealt round-robin over tiles, every chunk holds the same
 // number of probing tiles (+-1) at every tick, so the static split is balanced.
@@ -182,7 +193,9 @@ __device__ __noinline__ void gs_row_step_call(const GsDev* dp, const GsGlobals* 
 // column accesses).  The four 32-member groups of a probing tile go through the staged fast
 // path together — own columns, target gathers and commits are each issued for all four
 // before the first is consumed — so the tile pays two dependent memory latencies, not eight.
-// Whatever the fast path declines goes to the generic gs_row_step.
+// Every other group with activity is queued for the CTA's drain, where members with mail go through
+// the fast gossip tier (gs_fast_gossip) and whatever either fast path declines goes to the generic
+// gs_row_step.
 template <bool COORDS>
 __global__ void __launch_bounds__(GS_BLOCK, GS_MIN_BLOCKS)
     gs_tick_kernel(const __grid_constant__ GsDev d, const GsGlobals* __restrict__ gp, uint32_t k_off) {
@@ -374,9 +387,12 @@ __global__ void __launch_bounds__(GS_BLOCK, GS_MIN_BLOCKS)
     // which members of the group: mail, a probe action due (members the fast path finished have moved
     // their `due` on), or the push-pull ticker
     const uint32_t w = __ldcg(inbox_cur + i);
-    const bool a = w != 0u || __ldcg(d.due + i) == t ||
+    const bool due_now = __ldcg(d.due + i) == t;
+    const bool a = w != 0u || due_now ||
                    (g.pp_interval != 0u && gs_pp_due(g.pp_interval, g.rot_pp, i / g.phase_group, t));
-    if (a) gs_row_step_call<COORDS>(&d, gp, i, t, w, s_stat, s_heard, s_q);
+    // members with mail try the fast gossip tier first; whatever it declines takes the generic step
+    const bool fast = w != 0u && gs_fast_gossip_call<COORDS>(&d, gp, i, t, gslot, w, due_now, s_stat, s_heard, s_q);
+    if (a && !fast) gs_row_step_call<COORDS>(&d, gp, i, t, w, s_stat, s_heard, s_q);
   }
   __syncthreads();  // the queue is drained (and its counters may be reused two rounds from now)
   }  // rounds

@@ -891,17 +891,24 @@ GS_DEV bool gs_fast_target(const GsDev& d, const G& g, uint32_t cur, uint32_t i,
   return true;
 }
 
-// Returns true when the member was fully handled; *acked tells whether the direct probe
-// succeeded (stats: PROBES +1, ACKS +acked, ACTIVE_ROWS +1 are added by the caller).
-template <class G, class Sink>
-GS_DEV bool gs_fast_finish(const GsDev& d, const G& g, Sink& sink, uint32_t i, uint32_t t,
-                           const GsFastProbe& f, bool* acked) {
+// Stage C's decision alone (no write): can gs_fast_finish take this member?
+template <class G>
+GS_DEV bool gs_fast_accept(const G& g, uint32_t i, uint32_t t, const GsFastProbe& f) {
   const uint32_t rank = gs_key_rank(f.kc);
   if (gs_key_truth(f.kc) == GS_TRUTH_NONE || rank == GS_RANK_DEAD || rank == GS_RANK_LEFT ||
       gs_key_pending(f.kc))
     return false;  // ring entry must be skipped or needs the heard mask: generic path
   if (g.pp_interval != 0u && gs_pp_due(g.pp_interval, g.rot_pp, i / g.phase_group, t))
     return false;  // the push-pull ticker fires too: generic path
+  return true;
+}
+
+// Returns true when the member was fully handled; *acked tells whether the direct probe
+// succeeded (stats: PROBES +1, ACKS +acked, ACTIVE_ROWS +1 are added by the caller).
+template <class G, class Sink>
+GS_DEV bool gs_fast_finish(const GsDev& d, const G& g, Sink& sink, uint32_t i, uint32_t t,
+                           const GsFastProbe& f, bool* acked) {
+  if (!gs_fast_accept(g, i, t, f)) return false;
   uint32_t m = f.m;
   if (gs_key_truth(f.kc) == GS_TRUTH_UP && gs_extra(g, i, f.c) + gs_extra(g, f.c, i) <= g.T) {
     const uint32_t aw = gs_meta_aw(m);
@@ -918,5 +925,188 @@ GS_DEV bool gs_fast_finish(const GsDev& d, const G& g, Sink& sink, uint32_t i, u
   }
   d.cursor[i] = f.cursor + 1u;
   if (m != f.m) d.meta[i] = m;
+  return true;
+}
+
+// ---------------------------------------------------------------------------------------
+// Staged fast path for the bulk of a join cascade: a member that is up, listed alive,
+// established and clean, whose mail only repeats rumors it has heard or brings fresh alive /
+// join-intent / leave-intent rumors, and which may have its gossip turn and its probe ticker
+// at the same tick.  Same order as gs_row_step — A (accept), C (probe), D (gossip), E (wake) —
+// with two rounds of loads instead of about five dependent ones: (A) the member's own columns,
+// (B) the status gathers of the four gossip candidates of the first Philox block and of the
+// probe target, with the retransmit counters of the queued broadcasts.  Nothing is written
+// before every condition has held; a member that does not qualify is left untouched and takes
+// gs_row_step.  Declined (generic step): packet loss, CSR graphs, latency pools, push-pull, a
+// byte budget that can bind, tracked broadcasts in more than GS_FG_PAIRS counter pairs (GS_TX:
+// two slots share one 16-bit element), accusations, user events
+// and update rumors (event windows, logging), watched members with fresh mail, a probe action
+// other than the ticker of an idle member, gossip candidates that are pending joiners or dead
+// (those need the rumor table or change_tick), and a first block short of GossipNodes peers.
+// GSIM_FLAG_NO_FAST_GOSSIP (256) turns the tier off; results are identical either way.
+// ---------------------------------------------------------------------------------------
+#define GS_FG_PAIRS 4u  // retransmit-counter pairs the tier loads at once (up to 8 tracked broadcasts)
+
+GS_DEV uint32_t gs_popc(uint32_t x) {
+#if defined(__CUDA_ARCH__)
+  return __popc(x);
+#else
+  return (uint32_t)__builtin_popcount(x);
+#endif
+}
+GS_DEV uint32_t gs_lowbit(uint32_t x) {  // index of the lowest set bit of x != 0
+#if defined(__CUDA_ARCH__)
+  return __ffs(x) - 1;
+#else
+  return (uint32_t)__builtin_ctz(x);
+#endif
+}
+
+template <class Sink>
+GS_DEV bool gs_fast_gossip(const GsDev& d, const GsGlobals& g, Sink& sink, uint32_t i, uint32_t t, uint32_t gslot,
+                           uint32_t inb, bool due_now) {
+  const uint32_t am = g.active_mask;
+  uint32_t pm = 0;  // counter pairs holding a tracked slot
+  for (uint32_t x = am; x != 0u; x &= x - 1u) pm |= 1u << (gs_lowbit(x) >> 1);
+  if (inb == 0u || (inb & GS_ACC_BIT) || (g.flags & 256u) || g.loss_thr != 0u || g.graph_n != 0u || g.n_dcs != 0u ||
+      g.pp_interval != 0u || g.active_bytes > g.udp_avail || g.n < 2u || g.gossip_nodes == 0u ||
+      gs_popc(pm) > GS_FG_PAIRS)
+    return false;
+  const uint32_t cur = t & 1u;
+  const size_t cap = g.cap;
+
+  // ---- stage A: own columns (independent loads) ----
+  GsFastProbe f;
+  f.k = d.key[cur][i];
+  f.m = d.meta[i];
+  const uint32_t q0 = d.queued[i], heard0 = d.heard[i];
+  const uint32_t rbits = inb & ~(GS_ACC_BIT | GS_WAKE_BIT) & am;
+  const uint32_t lt0 = rbits != 0u ? d.ltime_member[i] : 0u;
+  if (due_now) {
+    f.cursor = d.cursor[i];
+    f.pass = d.pass[i];
+  }
+  const uint32_t m0 = f.m;
+  if (gs_key_truth(f.k) != GS_TRUTH_UP || gs_key_rank(f.k) != GS_RANK_ALIVE ||
+      (m0 & (GS_META_DIRTY | GS_META_ISOLATED | GS_META_LEAVING)) || (q0 & ~am))
+    return false;
+  if (due_now && gs_meta_stage(m0) != GS_STAGE_IDLE) return false;  // indirect probes, probe deadline
+  // section A: every fresh rumor is accepted (alive and intents have no drop rule)
+  const uint32_t fresh = rbits & ~heard0;
+  uint32_t lt = lt0;
+  if (fresh != 0u) {
+    if (m0 & GS_META_WATCHED) return false;  // join events are logged by the generic step
+    for (uint32_t fm = fresh; fm != 0u; fm &= fm - 1u) {
+      const GsRumor& ru = g.rumors[gs_lowbit(fm)];
+      if (ru.kind == GS_RUMOR_JOIN_INTENT || ru.kind == GS_RUMOR_LEAVE_INTENT) {
+        if (ru.ltime >= lt) lt = ru.ltime + 1u;  // clock.Witness
+      } else if (ru.kind != GS_RUMOR_ALIVE) {
+        return false;
+      }
+    }
+  }
+  const uint32_t q1 = q0 | fresh;
+  const bool gossip = gslot == gs_meta_gphase(m0) && q1 != 0u;
+
+  // ---- stage B: peer status gathers, retransmit counters ----
+  if (due_now && !gs_fast_target(d, g, cur, i, f)) return false;
+  uint32_t cc[4], kc[4], txw[2] = {0u, 0u};  // txw: the x-th pair of pm in bits 16x .. 16x + 15
+  if (gossip) {
+    const GsU4 blk = gs_philox(g.seed_lo, g.seed_hi, i, t, GS_PUR_GOSSIP, 0u);
+#pragma unroll
+    for (uint32_t x = 0; x < 4u; ++x) {
+      cc[x] = gs_fastmod(gs_u4_get(blk, x), g.n, g.n_magic);
+      kc[x] = cc[x] != i ? gs_peer_key(d, cur, cc[x], false) : 0u;
+    }
+    uint32_t mm = pm;
+#pragma unroll
+    for (uint32_t x = 0; x < GS_FG_PAIRS; ++x) {
+      if (mm != 0u) {
+        const uint32_t p = gs_lowbit(mm);
+        mm &= mm - 1u;
+        const uint32_t w = *reinterpret_cast<const uint16_t*>(d.tx + GS_TX(2u * p, cap, i));
+        txw[x >> 1] |= w << ((x & 1u) * 16u);
+      }
+    }
+  }
+  if (due_now && !gs_fast_accept(g, i, t, f)) return false;
+  // kRandomNodes (gs_krandom, mode 0) over the first block: tries = min(3n, 32) >= 6 covers all four draws
+  const uint32_t want = g.gossip_nodes > 8u ? 8u : g.gossip_nodes;
+  uint32_t np = 0, sel = 0;
+  if (gossip) {
+#pragma unroll
+    for (uint32_t x = 0; x < 4u; ++x) {
+      if (np < want) {
+        const uint32_t c = cc[x], k = kc[x], rank = gs_key_rank(k);
+        bool take = c != i && gs_key_truth(k) != GS_TRUTH_NONE && rank != GS_RANK_LEFT;
+        if (take && (rank == GS_RANK_DEAD || gs_key_pending(k))) return false;
+#pragma unroll
+        for (uint32_t y = 0; y < x; ++y) take = take && !(((sel >> y) & 1u) && cc[y] == c);
+        if (take) {
+          sel |= 1u << x;
+          ++np;
+        }
+      }
+    }
+    if (np < want) return false;
+  }
+
+  // ---- commit: what gs_row_step writes for this member ----
+  const uint32_t inxt = (t + 1u) & g.ring_mask;
+  sink.activity();
+  d.inbox[t & g.ring_mask][i] = 0u;
+  sink.stat(GS_ST_ACTIVE_ROWS, 1);
+  if (fresh != 0u) {
+    for (uint32_t fm = fresh; fm != 0u; fm &= fm - 1u) {
+      const uint32_t r = gs_lowbit(fm);
+      d.tx[GS_TX(r, cap, i)] = 0;  // queued with transmits = 0
+      sink.heard(r);
+    }
+    sink.stat(GS_ST_RUMORS_ACCEPTED, gs_popc(fresh));
+    d.heard[i] = heard0 | fresh;
+    if (lt != lt0) d.ltime_member[i] = lt;
+  }
+  if (due_now) {
+    bool acked = false;
+    (void)gs_fast_finish(d, g, sink, i, t, f, &acked);  // accepted above
+    sink.stat(GS_ST_PROBES, 1);
+    if (acked) sink.stat(GS_ST_ACKS, 1);
+  }
+  uint32_t q = q1;
+  if (gossip) {
+    // every packet carries the whole queue: broadcast r rides in packets 0 .. sends_r - 1,
+    // sends_r = min(np, max(1, limit - transmits_r)) (gs_row_step section D)
+    const uint32_t lim = g.retransmit_limit;
+    uint32_t pk0 = 0, pk1 = 0, pk2 = 0, pk3 = 0, n_pkts = 0, sent = 0;
+    for (uint32_t qm = q1; qm != 0u; qm &= qm - 1u) {
+      const uint32_t r = gs_lowbit(qm), x = gs_popc(pm & ((1u << (r >> 1)) - 1u));  // r's pair in txw
+      const uint32_t tx = (fresh >> r) & 1u ? 0u : ((x >> 1 ? txw[1] : txw[0]) >> ((x & 1u) * 16u + (r & 1u) * 8u)) & 0xFFu;
+      const uint32_t room = lim > tx ? lim - tx : 1u;
+      const uint32_t s = room < np ? room : np;
+      d.tx[GS_TX(r, cap, i)] = (uint8_t)(tx + s);
+      if (tx + s >= lim) q &= ~(1u << r);  // broadcast finished
+      sent += s;
+      if (s > n_pkts) n_pkts = s;
+      pk0 |= 1u << r;
+      pk1 |= s > 1u ? 1u << r : 0u;
+      pk2 |= s > 2u ? 1u << r : 0u;
+      pk3 |= s > 3u ? 1u << r : 0u;
+    }
+    sink.stat(GS_ST_RUMORS_SENT, sent);
+    sink.stat(GS_ST_GOSSIP_PACKETS, n_pkts);
+    // packet q goes to the q-th peer taken: the selected candidates in draw order
+#pragma unroll
+    for (uint32_t x = 0; x < 4u; ++x) {
+      if ((sel >> x) & 1u) {
+        if (pk0 != 0u) gs_post(d, g, sink, inxt, cc[x], pk0);
+        pk0 = pk1;
+        pk1 = pk2;
+        pk2 = pk3;
+        pk3 = 0u;
+      }
+    }
+  }
+  if (q != q0) d.queued[i] = q;
+  if (q != 0u) gs_post(d, g, sink, inxt, i, GS_WAKE_BIT);
   return true;
 }

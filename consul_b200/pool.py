@@ -23,6 +23,7 @@ FLAG_NO_GRAPH = 2
 FLAG_NO_WINDOWS = 16
 FLAG_PUSH_PULL = 32
 FLAG_COORDINATES = 64
+FLAG_NO_FAST_GOSSIP = 256
 MEMBER_WATCHED = 1
 
 

@@ -159,6 +159,10 @@ typedef struct gsim_config {
  * trip (0.5 ms + the latency matrix there and back) and the target's coordinate.  348 B per
  * member; single-GPU pools.  IEEE double arithmetic, bit-identical to the oracle. */
 #define GSIM_FLAG_COORDINATES 64u
+/* Run every member with mail through the generic row step, without the fast gossip tier (DESIGN.md
+ * 4.1): for measurements and for tests that compare the two.  Same results either way.  The
+ * environment variable GSIM_NO_FAST_GOSSIP does the same for every pool of the process. */
+#define GSIM_FLAG_NO_FAST_GOSSIP 256u
 
 /* Preset defaults.  LAN/WAN: [U] memberlist DefaultLANConfig/DefaultWANConfig as
  * pinned by agent/config/runtime.go:1271-1413 with Consul's overrides
